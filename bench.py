@@ -27,6 +27,14 @@ embarrassingly; no collective on the data path) -> weak scaling; time = max over
 
 `--impl reference` times only the CPU runner: a step is one pass of every runner over its 4 chunks; W warm-up passes,
 then exactly K timed passes, value = samples of the K passes / their wall time.
+
+`--steps K` / `--warmup W` apply to every timed run: the flagship and, in the default run, the hac / sup sub-results
+and their auto-batch runs (device-resident and e2e loops alike).
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed e2e step returned to its caller for each model
+timed (the flagship, plus hac and sup in the default run): DIR/<model>_{moves,sequence,qstring,n_bases,chunk_index}.npy
+in float32.  DIR must be new or empty.  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output.  Not available with `--impl reference`, whose timed passes discard their outputs.
 """
 from __future__ import annotations
 
@@ -51,10 +59,11 @@ MODELS = {
 }
 # SURVEY.md section 8(d): algorithmic FLOP per input sample
 FLOP_PER_SAMPLE = {"fast": 0.1435e6, "hac": 2.139e6, "sup": 14.35e6}
-SUB_MODELS = {"hac": dict(batch=512, steps=8), "sup": dict(batch=128, steps=6)}
+SUB_MODELS = {"hac": dict(batch=512), "sup": dict(batch=128)}
 NUM_SMS = 148
 DEFAULT_RUNNERS = {"fast": 4, "hac": 4, "sup": 2}   # batches in flight per GPU (dorado's --num-runners; see --runners)
 METRIC = "basecalled samples/s"
+DUMP_LIMIT = 64 << 20   # bytes of .npy data one --dump-outputs directory may receive
 
 
 def model_dir(kind):
@@ -285,7 +294,25 @@ def kernel_work(cfg, kind, N, T, T_out):
     return work
 
 
-def bench_b200(kind, batch, chunksize, steps, warmup, R, rank, local_rank, world, sampler=None, want_cpu=False):
+def dump_outputs(out_dir, kind, result, budget):
+    """One step's call_chunks_raw result (moves, sequence, qstring [N, T_out] uint8; n_bases [N]) as float32 .npy files.
+    Sequence and qstring are zeroed past each chunk's n_bases: a caller's DecodedChunk ends there and the rest of the
+    buffer is not part of the result.  Above `budget` bytes, a fixed seeded sample of chunks is written; chunk_index
+    lists the chunks kept."""
+    moves, seq, qs, nb = (np.array(a) for a in result)
+    N, T = moves.shape
+    valid = np.arange(T)[None, :] < nb[:, None]
+    seq, qs = np.where(valid, seq, 0), np.where(valid, qs, 0)
+    keep = min(N, max(1, budget // (3 * T * 4 + 8)))
+    rows = np.arange(N) if keep == N else np.sort(np.random.default_rng(0).choice(N, keep, replace=False))
+    out_dir = pathlib.Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in (("moves", moves), ("sequence", seq), ("qstring", qs), ("n_bases", nb), ("chunk_index", np.arange(N))):
+        np.save(out_dir / f"{kind}_{name}.npy", a[rows].astype(np.float32))
+
+
+def bench_b200(kind, batch, chunksize, steps, warmup, R, rank, local_rank, world, sampler=None, want_cpu=False,
+               dump=None, dump_budget=DUMP_LIMIT):
     import torch
     import torch.distributed as dist
     from dorado_b200.config import load_model_config
@@ -354,6 +381,8 @@ def bench_b200(kind, batch, chunksize, steps, warmup, R, rank, local_rank, world
     run_calls(steps)
     barrier()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
+    if dump is not None and rank == 0:
+        dump_outputs(dump, kind, last[(steps - 1) % R], dump_budget)   # step i ran on runner i % R
     bases_last = int(next(c for c in last if c is not None)[3][:N].sum())
     e2e_value = world * samples_per_step * steps / e2e_s
     h2d = N * T * 2
@@ -468,7 +497,18 @@ def main():
                          "chains; four batches side by side fill the SMs, profiles/r02_b11_*), 2 for hac and sup")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU reference leg (batch sweeps)")
     ap.add_argument("--no-sub-models", action="store_true", help="skip the hac@512 / sup@128 sub-results of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned (moves, sequence, qstring, n_bases) "
+                         "as DIR/<model>_<name>.npy, float32, at most 64 MB in all; DIR must be new or empty")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None:
+        if args.impl == "reference":
+            ap.error("--dump-outputs records the B200 path; the reference arm's timed passes return no outputs")
+        d = pathlib.Path(args.dump_outputs)
+        if d.exists() and (not d.is_dir() or any(d.iterdir())):
+            ap.error(f"--dump-outputs {d}: must be a new or empty directory, so that no earlier run's files mix in")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -503,13 +543,15 @@ def main():
     time.sleep(0.3)  # let nvidia-smi reach its sampling loop
     R = max(1, args.runners if args.runners is not None else DEFAULT_RUNNERS[kind])
     config["runners_per_gpu"] = R
-    main_res = bench_b200(kind, args.batch, args.chunksize, args.steps, args.warmup, R, rank, local_rank, world, sampler=sampler,
-                          want_cpu=(world == 1 and not args.no_cpu_baseline))
-    subs = {}
     default_run = kind == "fast" and args.batch == 512 and not args.no_sub_models
+    dump_budget = DUMP_LIMIT // (1 + len(SUB_MODELS) if default_run else 1)
+    main_res = bench_b200(kind, args.batch, args.chunksize, args.steps, args.warmup, R, rank, local_rank, world, sampler=sampler,
+                          want_cpu=(world == 1 and not args.no_cpu_baseline), dump=args.dump_outputs, dump_budget=dump_budget)
+    subs = {}
     if default_run:
         for sk, sc in SUB_MODELS.items():
-            res = bench_b200(sk, sc["batch"], args.chunksize, sc["steps"], 3, DEFAULT_RUNNERS[sk], rank, local_rank, world)
+            res = bench_b200(sk, sc["batch"], args.chunksize, args.steps, args.warmup, DEFAULT_RUNNERS[sk], rank, local_rank, world,
+                             dump=args.dump_outputs, dump_budget=dump_budget)
             if rank == 0:
                 keep = ("value", "ms_per_step", "steps", "e2e", "forward_ms_per_step", "decode_ms_per_step", "batch_per_gpu",
                         "chunk_samples", "runners_per_gpu", "gpu_launches", "bases_called_last_step")
@@ -531,7 +573,8 @@ def main():
                                                          num_runners=DEFAULT_RUNNERS[sk])
             probe.close()
             auto_batch = int(dims[0][0])
-            res = bench_b200(sk, auto_batch, args.chunksize, max(3, sc["steps"] // 2), 3, DEFAULT_RUNNERS[sk], rank, local_rank, world)
+            res = bench_b200(sk, auto_batch, args.chunksize, args.steps, args.warmup, DEFAULT_RUNNERS[sk], rank, local_rank,
+                             world)
             if rank == 0:
                 subs[sk + "_auto_batch"] = {k: res[k] for k in ("value", "ms_per_step", "steps", "e2e", "batch_per_gpu",
                                                                "chunk_samples", "runners_per_gpu", "gpu_launches")}

@@ -1,7 +1,9 @@
 """Front end of the hot path (SURVEY.md 8f rows 2-3) on the CPU: the product's host logic (generate_chunks,
 stitch_chunks through the C ABI) and the numpy oracle of the device-side scaling, both pinned to
   * the golden vectors of the reference's own tests (tests/ChunkTest.cpp, tests/StitchTest.cpp), restated below,
-  * the compiled reference (oracle/_ref: chunk.cpp, stitch.cpp, tensor_utils.cpp) on random inputs,
+  * the compiled reference (chunk.cpp, stitch.cpp, tensor_utils.cpp) on seeded random inputs, whose outputs
+    tools/make_golden_reference.py records as digests in tests/golden/reference_cpu.npz (the *_cases functions below
+    generate the inputs for both),
   * the committed fixture tests/golden/frontend.npz (generated from the compiled reference).
 """
 import numpy as np
@@ -11,6 +13,12 @@ from conftest import ROOT
 from dorado_b200 import lib as L
 from dorado_b200.frontend import generate_chunks, stitch_chunks
 from oracle import frontend_oracle as fo
+from oracle.golden import digest
+
+
+@pytest.fixture(scope="module")
+def golden():
+    return np.load(ROOT / "tests" / "golden" / "reference_cpu.npz")
 
 
 # ---- generate_chunks -------------------------------------------------------------------------------------------
@@ -49,18 +57,27 @@ def test_generate_chunks_properties_of_ChunkTest(chunk_size, stride, overlap):
         assert offs == fo.generate_chunks(int(num_samples), chunk_size, stride, overlap)
 
 
-def test_generate_chunks_matches_compiled_reference(reference):
+def generate_chunks_cases():
     rng = np.random.default_rng(7)
     for _ in range(300):
         stride = int(rng.choice([1, 5, 6, 12]))
         chunk = stride * int(rng.integers(2, 400))
         overlap = stride * int(rng.integers(0, chunk // stride))
         n = int(rng.integers(1, 40 * chunk))
-        want = reference.generate_chunks(n, chunk, stride, overlap)
-        assert generate_chunks(n, chunk, stride, overlap) == want
-        assert fo.generate_chunks(n, chunk, stride, overlap) == want
-    with pytest.raises(RuntimeError):
-        reference.generate_chunks(0, 9996, 6, 498)
+        yield n, chunk, stride, overlap
+
+
+def test_generate_chunks_matches_compiled_reference(golden):
+    want = golden["generate_chunks"]
+    cases = list(generate_chunks_cases())
+    assert len(cases) == len(want)
+    for args, w in zip(cases, want):
+        got = generate_chunks(*args)
+        assert (digest(np.array(got, np.uint64)) == w).all(), args
+        assert fo.generate_chunks(*args) == got
+    assert golden["generate_chunks_zero_raises"]   # the reference throws on an empty read; so must the product
+    with pytest.raises(L.B200Error):
+        generate_chunks(0, 9996, 6, 498)
 
 
 def test_generate_chunks_capacity_reports_full_count():
@@ -111,20 +128,30 @@ def _random_called_read(rng, n_samples, chunk, stride, overlap):
     return chunks
 
 
-def test_stitch_chunks_matches_compiled_reference(reference):
+def stitch_cases():
     rng = np.random.default_rng(11)
-    for it in range(200):
+    for _ in range(200):
         stride = int(rng.choice([1, 5, 6]))
         chunk = stride * int(rng.integers(8, 120))
         overlap = stride * int(rng.integers(0, max(1, chunk // stride // 2)))
         n = int(rng.integers(1, 12 * chunk))
-        chunks = _random_called_read(rng, n, chunk, stride, overlap)
-        want = reference.stitch_chunks(chunks, n, stride)
+        yield n, chunk, stride, overlap, _random_called_read(rng, n, chunk, stride, overlap)
+
+
+def stitch_digest(seq, q, moves):
+    return digest(seq, q, np.asarray(moves, np.uint8))
+
+
+def test_stitch_chunks_matches_compiled_reference(golden):
+    want = golden["stitch_chunks"]
+    cases = list(stitch_cases())
+    assert len(cases) == len(want)
+    for it, ((n, chunk, stride, overlap, chunks), w) in enumerate(zip(cases, want)):
         for impl in (stitch_chunks, fo.stitch_chunks):
             seq, q, moves = impl(chunks, n, stride)
-            assert (seq, q) == want[:2] and moves.tolist() == want[2].tolist(), (it, n, chunk, stride, overlap)
-        assert len(want[2]) == n // stride or len(chunks) > 1
-        assert int(want[2].sum()) == len(want[0])
+            assert (stitch_digest(seq, q, moves) == w).all(), (it, n, chunk, stride, overlap)
+        assert len(moves) == n // stride or len(chunks) > 1
+        assert int(moves.sum()) == len(seq)
 
 
 def test_stitch_chunks_rejects_bad_input():
@@ -142,29 +169,41 @@ def test_stitch_chunks_rejects_bad_input():
 
 
 # ---- raw int16 -> scaled, repeat-padded fp16 rows (numpy oracle of the device kernel) -----------------------------
-def test_scaling_oracle_like_TensorUtilsTest(reference):
+def scaling_cases():
     # tests/TensorUtilsTest.cpp:121-143: random sizes < 100, shift in [-100, 100], scale in [0.1, 100], zero tolerance
     rng = np.random.default_rng(42)
     for _ in range(40):
         n = int(rng.integers(1, 100))
         shift, scale = float(rng.uniform(-100, 100)), float(rng.uniform(0.1, 100))
-        raw = (rng.random(n) * 1000).astype(np.int16)
-        want = reference.make_chunk_input(raw, 0, n, shift, scale)
+        yield (rng.random(n) * 1000).astype(np.int16), shift, scale
+
+
+def test_scaling_oracle_like_TensorUtilsTest(golden):
+    want = golden["scaling"]
+    cases = list(scaling_cases())
+    assert len(cases) == len(want)
+    for (raw, shift, scale), w in zip(cases, want):
         got = fo.scale_i16_to_f16(raw, np.float32(shift), np.float32(scale))
-        assert (got.view(np.uint16) == want.view(np.uint16)).all()
+        assert (digest(got.view(np.uint16)) == w).all()
 
 
-def test_chunk_input_oracle_matches_compiled_reference(reference):
+def chunk_input_cases():
     rng = np.random.default_rng(5)
     for _ in range(60):
         chunk = 6 * int(rng.integers(2, 300))
         n = int(rng.integers(1, 6 * chunk))
         raw = rng.integers(-32768, 32768, n).astype(np.int16)
         shift, scale = float(rng.uniform(-500, 900)), float(rng.uniform(0.5, 400))
-        for off in fo.generate_chunks(n, chunk, 6, 6 * int(rng.integers(0, chunk // 12 + 1))):
-            want = reference.make_chunk_input(raw, off, chunk, shift, scale)
-            got = fo.chunk_input(raw, off, chunk, shift, scale)
-            assert (got.view(np.uint16) == want.view(np.uint16)).all()
+        yield raw, fo.generate_chunks(n, chunk, 6, 6 * int(rng.integers(0, chunk // 12 + 1))), chunk, shift, scale
+
+
+def test_chunk_input_oracle_matches_compiled_reference(golden):
+    want = golden["chunk_input"]
+    cases = list(chunk_input_cases())
+    assert len(cases) == len(want)
+    for (raw, offs, chunk, shift, scale), w in zip(cases, want):
+        rows = [fo.chunk_input(raw, off, chunk, shift, scale).view(np.uint16) for off in offs]
+        assert (digest(*rows) == w).all()
 
 
 def test_frontend_golden_fixture_matches_oracle():
@@ -231,32 +270,49 @@ def test_select_batch_size_rejects_bad_tables():
 
 
 # ---- generate_variable_chunks (first piece of SURVEY 8f row 1) -------------------------------------------------------
-def test_generate_variable_chunks_like_ChunkTest(reference):
-    from dorado_b200.frontend import generate_variable_chunks
-    for args in [(0, 9996, 6, 498), (12345, 0, 6, 498), (12345, 9996, 0, 498), (12345, 9996, 10, 498), (12345, 6, 6, 498),
-                 (12345, 9996, 7, 498), (12345, 9996, 7, 0), (12345, 9996, 6, 9996), (12345, 9996, 6, 9997)]:
-        with pytest.raises(L.B200Error):
-            generate_variable_chunks(*args)
-        with pytest.raises(RuntimeError):
-            reference.generate_variable_chunks(*args)
-    golden = [((9996 // 2, 9996, 6, 498), [(0, 4998)]), ((9996, 9996, 6, 498), [(0, 9996)]),
-              ((9996 + 1, 9996, 6, 498), [(0, 5244), (4752, 9997)]),
-              ((9996 + 9996 // 2, 9996, 6, 498), [(0, 7746), (7248, 14994)]),
-              ((2 * 9996 + 9996 // 2, 9996, 1, 0), [(0, 8330), (8330, 16660), (16660, 24990)]),
-              ((3 * 9996, 9996, 6, 498), [(0, 7866), (7374, 15240), (14748, 22614), (22122, 29988)])]
-    for args, want in golden:
-        assert generate_variable_chunks(*args) == want == fo.generate_variable_chunks(*args) == reference.generate_variable_chunks(*args)
+VARIABLE_CHUNKS_INVALID = [(0, 9996, 6, 498), (12345, 0, 6, 498), (12345, 9996, 0, 498), (12345, 9996, 10, 498),
+                           (12345, 6, 6, 498), (12345, 9996, 7, 498), (12345, 9996, 7, 0), (12345, 9996, 6, 9996),
+                           (12345, 9996, 6, 9997)]
+VARIABLE_CHUNKS_GOLDEN = [((9996 // 2, 9996, 6, 498), [(0, 4998)]), ((9996, 9996, 6, 498), [(0, 9996)]),
+                          ((9996 + 1, 9996, 6, 498), [(0, 5244), (4752, 9997)]),
+                          ((9996 + 9996 // 2, 9996, 6, 498), [(0, 7746), (7248, 14994)]),
+                          ((2 * 9996 + 9996 // 2, 9996, 1, 0), [(0, 8330), (8330, 16660), (16660, 24990)]),
+                          ((3 * 9996, 9996, 6, 498), [(0, 7866), (7374, 15240), (14748, 22614), (22122, 29988)])]
+
+
+def variable_chunks_cases():
     rng = np.random.default_rng(42)
     for chunk_size, stride, overlap in [(9996, 6, 498), (9996, 7, 497), (9996, 12, 492), (9996, 17, 510), (555, 5, 25),
                                         (83, 1, 13), (123, 1, 0)]:
         for n in rng.integers(1024, 2097152, 16):
-            iv = generate_variable_chunks(int(n), chunk_size, stride, overlap)
-            assert iv == reference.generate_variable_chunks(int(n), chunk_size, stride, overlap)
-            assert iv == fo.generate_variable_chunks(int(n), chunk_size, stride, overlap)
-            assert iv[0][0] == 0 and iv[-1][1] == n
-            assert all(a % stride == 0 for a, _ in iv[1:]) and all(b % stride == 0 for _, b in iv[:-1])
-            assert all(0 < b - a <= chunk_size for a, b in iv)
-            assert all(iv[i - 1][1] - iv[i][0] <= overlap for i in range(1, len(iv)))
+            yield int(n), chunk_size, stride, overlap
+
+
+def intervals_digest(iv):
+    return digest(np.array(iv, np.uint64).reshape(-1, 2))
+
+
+def test_generate_variable_chunks_like_ChunkTest(golden):
+    from dorado_b200.frontend import generate_variable_chunks
+    assert golden["variable_chunks_invalid_raises"].all()   # the reference throws on every one of these
+    for args in VARIABLE_CHUNKS_INVALID:
+        with pytest.raises(L.B200Error):
+            generate_variable_chunks(*args)
+    assert len(golden["variable_chunks_golden"]) == len(VARIABLE_CHUNKS_GOLDEN)
+    for (args, want), w in zip(VARIABLE_CHUNKS_GOLDEN, golden["variable_chunks_golden"]):
+        assert generate_variable_chunks(*args) == want == fo.generate_variable_chunks(*args)
+        assert (intervals_digest(want) == w).all()
+    want = golden["variable_chunks"]
+    cases = list(variable_chunks_cases())
+    assert len(cases) == len(want)
+    for (n, chunk_size, stride, overlap), w in zip(cases, want):
+        iv = generate_variable_chunks(n, chunk_size, stride, overlap)
+        assert (intervals_digest(iv) == w).all(), (n, chunk_size, stride, overlap)
+        assert iv == fo.generate_variable_chunks(n, chunk_size, stride, overlap)
+        assert iv[0][0] == 0 and iv[-1][1] == n
+        assert all(a % stride == 0 for a, _ in iv[1:]) and all(b % stride == 0 for _, b in iv[:-1])
+        assert all(0 < b - a <= chunk_size for a, b in iv)
+        assert all(iv[i - 1][1] - iv[i][0] <= overlap for i in range(1, len(iv)))
 
 
 def test_batch_size_granularity_like_the_reference():

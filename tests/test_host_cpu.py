@@ -202,12 +202,11 @@ def test_adapter_header_compiles_against_reference_headers():
     """include/B200ModelRunner.h implements dorado::basecall::ModelRunnerBase; type-check it against the
     reference's own headers where the reference tree is available (not on the GPU box)."""
     d = pathlib.Path("/root/reference/dorado")
-    if not d.exists():
+    if not os.path.isdir(d):   # also False where the tree exists but this user may not read it
         pytest.skip("reference tree not present")
     import torch
     t = pathlib.Path(torch.__file__).parent
     src = ROOT / "tests" / "data" / "adapter_check.cpp"
-    src.write_text('#include "B200ModelRunner.h"\nint main() { return 0; }\n')
     inc = [ROOT / "include", d, d / "basecall", d / "basecall/include", d / "nn/include", d / "config/include",
            d / "torch_utils/include", d / "utils/include", d / "models/include", d / "3rdparty/spdlog/include",
            d / "3rdparty/NVTX/c/include", d / "3rdparty/toml11/include"]
